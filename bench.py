@@ -4,6 +4,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  ... --dump-outputs DIR     also writes the weights and loss history of the timed run as DIR/<name>.npy
 
 A "step" is one outer AGD iteration (AGD.scala:237-332) = the reference's 3 + 2b applySmooth evaluations
 (flags = 0: every evaluation is executed; the history evaluation of :304 shares one sweep over X with the next
@@ -57,7 +58,25 @@ def parse():
     ap.add_argument("--parity-iters", type=int, default=10,
                     help="iterations of the full-size oracle comparison reported as `parity` (0 = off; on by default for "
                          "fp32 logistic workloads whose host copy is <= 64 GB)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed run returned (weights, loss history) as "
+                         "DIR/<name>.npy in float64, so that two builds can be compared output for output")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes each array as out_dir/<name>.npy in float64.  An array larger than its share of DUMP_BYTES is replaced by the
+    same seeded sample of its entries on every run, so that dumps of two builds stay comparable entry for entry."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64).ravel()
+        if a.nbytes > share:
+            a = a[np.sort(np.random.default_rng(SEED).choice(a.size, share // a.itemsize, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peaks():
@@ -217,7 +236,8 @@ def cpu_reference(rows: int, d: int, steps: int, warmup: int, repeats: int = 3):
                       f"{repeats} timed runs, {cores} partitions on {cores} pinned threads (fastest of the calibrated thread "
                       f"counts {cands} on this {ncpu}-thread host), first-touch placement, fp32 rows upcast to fp64",
             "host_threads": ncpu, "cgroup_cpu_quota": quota, "thread_calibration_examples_per_sec": calib,
-            "seconds": dt, "runs_seconds": runs, "iters_per_sec": r.iterations / dt, "passes": r.passes, "rows": rows}
+            "seconds": dt, "runs_seconds": runs, "iters_per_sec": r.iterations / dt, "passes": r.passes, "rows": rows,
+            "weights": r.weights, "loss_history": r.loss_history}
 
 
 def run_reference(args):
@@ -225,9 +245,11 @@ def run_reference(args):
     if rank != 0:
         return
     rows = cpu_sample_rows(args)
-    steps = max(1, min(args.steps, 4))        # each step is a bounded sample; keep the arm within minutes
+    steps = args.steps
     warm = 1 if args.warmup > 0 else 0
     res = cpu_reference(rows, args.dim, steps, warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"weights": res["weights"], "loss_history": res["loss_history"]})
     line = {
         "impl": "reference", "metric": METRIC, "value": res["value"], "unit": "examples/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": warm, "ms_per_step": res["seconds"] / steps * 1e3, "higher_is_better": True,
@@ -312,6 +334,8 @@ def run_b200(args):
     barrier()
     t1 = time.time()
     clocks = sampler.stop(t0, t1) if sampler else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"weights": w, "loss_history": hist})
     dev_s = max_over_ranks(st.device_ms_total / 1e3)
     value = total_rows * st.passes / dev_s
     # the bit-identical memoised pass structure (AGD_FLAG_MEMOIZE_FX), reported beside the headline; like the headline it gets

@@ -47,11 +47,32 @@ def test_reference_arm_uses_every_host_thread_under_torchrun():
     assert cb["host_threads"] == n and cb["cores"] in (n, max(1, n // 2), max(1, n // 4)) and len(cb["runs_seconds"]) == 3
 
 
+def load_dump(out_dir):
+    import numpy as np
+    return {n: np.load(os.path.join(out_dir, f"{n}.npy")) for n in ("weights", "loss_history")}
+
+
+def test_reference_arm_dumps_the_outputs_of_every_step(tmp_path):
+    """--steps sets the number of timed iterations; --dump-outputs writes what the timed run returned, the same on every run."""
+    for k in ("a", "b"):
+        lines = run_bench("--impl", "reference", "--steps", "6", "--warmup", "0", "--cpu-rows", "20000", "--dim", "64",
+                          "--dump-outputs", str(tmp_path / k))
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == 6
+    a, b = load_dump(tmp_path / "a"), load_dump(tmp_path / "b")
+    assert a["weights"].shape == (64,) and a["loss_history"].shape == (6,)
+    for n in a:
+        assert a[n].dtype == b[n].dtype == "float64" and (a[n] == b[n]).all()
+
+
 @pytest.mark.gpu
-def test_b200_arm_prints_the_contract_line():
-    lines = run_bench("--rows", "400000", "--steps", "4", "--warmup", "3", "--cpu-rows", "20000")
+def test_b200_arm_prints_the_contract_line(tmp_path):
+    lines = run_bench("--rows", "400000", "--steps", "4", "--warmup", "3", "--cpu-rows", "20000",
+                      "--dump-outputs", str(tmp_path))
     assert len(lines) == 1
     j = json.loads(lines[0])
+    out = load_dump(tmp_path)
+    assert out["weights"].shape == (1024,) and out["weights"].dtype == "float64" and out["loss_history"].shape == (4,)
+    assert out["loss_history"][-1] == j["final_loss"]
     assert BASE_KEYS | {"roofline", "clocks"} <= set(j) and "impl" not in j
     assert j["n_gpus"] == 1 and j["steps"] == 4 and j["warmup"] == 3 and j["dtype"] == "f64" and j["data"] == "synthetic"
     assert j["scaling"] in ("strong", "weak") and j["vs_baseline"] is None and j["value"] > 0 and j["gpu_launches"] > 0

@@ -1,5 +1,5 @@
 """Pins the CPU oracle against every test the reference's own suite holds for this path
-(/root/reference/src/test/scala/.../AcceleratedGradientDescentSuite.scala, cited as Suite.scala)
+(staple/spark-agd's src/test/scala/.../AcceleratedGradientDescentSuite.scala, cited as Suite.scala)
 and against the one Java known-answer value available (java.util.Random(42).nextGaussian()).
 
 The reference ships no golden vectors; tests/golden/reference_suite_anchors.json holds the values
